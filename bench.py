@@ -36,6 +36,29 @@ CONV3_FLOP = {  # per full-resolution patch voxel, 3x3x3 layers only (by kernel 
 }
 
 
+DUMP_SEED = 20260922
+DUMP_VOXELS = 1 << 21   # spatial positions sampled for --dump-outputs: C x 2^21 float32 (24 MB for 3 channels)
+
+
+def dump_outputs(directory, out):
+    """Writes the affinity map a caller of the timed path receives, as float32 .npy files under `directory`:
+    affinity_voxels.npy  (C, 2^21): every channel at a fixed, seeded, sorted set of flat zyx positions (drawn with
+                         replacement from np.random.default_rng(DUMP_SEED), so it depends only on the output shape)
+    affinity_plane.npy   (C, Y, X): the whole z plane in the middle of the chunk (every patch seam in y and x).
+    `out` is a (C, Z, Y, X) float32 torch tensor (on the GPU: only the sample leaves the device) or numpy array."""
+    os.makedirs(directory, exist_ok=True)
+    c, z = out.shape[0], out.shape[1]
+    idx = np.sort(np.random.default_rng(DUMP_SEED).integers(0, int(np.prod(out.shape[1:])), DUMP_VOXELS))
+    if isinstance(out, np.ndarray):
+        voxels, plane = out.reshape(c, -1)[:, idx], out[:, z // 2]
+    else:
+        import torch
+        voxels = out.reshape(c, -1)[:, torch.from_numpy(idx).to(out.device)].cpu().numpy()
+        plane = out[:, z // 2].cpu().numpy()
+    np.save(os.path.join(directory, "affinity_voxels.npy"), np.ascontiguousarray(voxels, dtype=np.float32))
+    np.save(os.path.join(directory, "affinity_plane.npy"), np.ascontiguousarray(plane, dtype=np.float32))
+
+
 def patch_count(chunk, patch, overlap):
     n = 1
     for c, p, o in zip(chunk, patch, overlap):
@@ -279,6 +302,8 @@ def main():
     ap.add_argument("--no-alt-precision", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed sample of what the last timed step "
+                    "computed to DIR/*.npy (rank 0; see dump_outputs), to compare two builds output for output")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", 0))
@@ -306,6 +331,8 @@ def main():
             r = ref.run(chunk_shape, per_step if timed else 1, 20260922 + i)   # a warm-up step is one patch
             if timed:
                 runs.append(r)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, runs[-1]["output"])
         agg = dict(seconds=sum(r["seconds"] for r in runs), patches=sum(r["patches"] for r in runs), sub=runs[0]["sub"],
                    parts={k: sum(r["parts"][k] for r in runs) for k in runs[0]["parts"]})
         agg["sub"] = (runs[0]["sub"][0] * len(runs),) + tuple(runs[0]["sub"][1:])   # voxels of all timed sub-chunks
@@ -375,6 +402,8 @@ def main():
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:   # before the profiled step below overwrites d_out
+        dump_outputs(args.dump_outputs, d_out)
     launches = eng.last_timing()["launches"]
     value = nvox * world * args.steps / (ms / 1e3) / 1e6
 

@@ -6,9 +6,9 @@ Plain numpy restatements, each citing the reference file:line it follows, of
   * ``Chunk.crop_margin``          chunk/base.py:691-726       (downstream)
   * ``AffinityMap.quantize``       chunk/affinity_map/base.py:33-57 (downstream: affinity -> uint8 image)
 
-Pinning: ``tests/test_oracle_vs_reference.py`` runs the REAL reference classes (imported from /root/reference by
-``oracle/reference_harness.py``) against these functions, bit-exact; ``tests/golden/operators.npz`` holds outputs of the
-real reference (``tests/golden/make_golden.py``) for the boxes where /root/reference is absent.
+Pinning, bit-exact: ``tests/test_operators_oracle.py`` compares these functions with outputs of the REAL reference
+classes, ``tests/golden/operators.npz`` (``tests/golden/make_golden_operators.py``) and, on fresh random inputs,
+``tests/golden/reference_pins.*`` (``tests/golden/make_golden_reference.py``).
 
 Reference quirks restated literally (the product mirrors them and DESIGN.md lists them):
   * ``normalize_contrast(per_section=True)``: the whole-array branch is the ``else`` clause of the ``for`` loop over

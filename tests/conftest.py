@@ -32,6 +32,13 @@ def golden():
 
 
 @pytest.fixture(scope="session")
+def pins():
+    """What the original chunkflow computed on the pinning tests' inputs (tests/reference_pins.py)."""
+    from reference_pins import Pins
+    return Pins()
+
+
+@pytest.fixture(scope="session")
 def unet_model():
     from chunkflow_b200.lib import load_source
     return load_source(MODEL_FILE).load_model(None)

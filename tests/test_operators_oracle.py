@@ -1,15 +1,12 @@
 """Pins oracle/operators_oracle.py (SURVEY.md section 8 f3) to golden vectors made by the REAL reference
-(tests/golden/make_golden_operators.py) and, where /root/reference exists, to the reference classes on fresh random inputs."""
-import io
+(tests/golden/make_golden_operators.py) and to what the reference classes computed on fresh random inputs
+(tests/golden/make_golden_reference.py)."""
 import os
-import warnings
-from contextlib import redirect_stderr, redirect_stdout
 
 import numpy as np
 import pytest
 
 from oracle import operators_oracle as OP
-from oracle import reference_harness as H
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "operators.npz")
 
@@ -52,51 +49,45 @@ def test_quantize_maskout_crop_golden(gold):
         OP.crop_margin(gold["aff"], (0, 0, 0), (1, 2))
 
 
-@pytest.mark.skipif(not H.available(), reason="/root/reference not present (GPU box)")
-@pytest.mark.parametrize("seed", [0, 1, 2])
-def test_against_real_reference(seed):
-    _, Chunk, _ = H.import_reference()
-    warnings.simplefilter("ignore")
-    from chunkflow.chunk.image.base import Image
-    from chunkflow.chunk.affinity_map import AffinityMap
+def real_reference_case(seed):
     rng = np.random.default_rng(seed)
     z, y, x = 5, 33, 47
     img = (rng.random((z, y, x)) ** (1 + seed) * rng.integers(60, 256)).astype(np.uint8)
     img[seed % z] //= 8
     lo, hi = [(0.01, 0.01), (0.1, 0.0), (0.0, 0.2)][seed]
-    im = Image(img.copy())
-    with redirect_stdout(io.StringIO()), redirect_stderr(io.StringIO()):
-        im.normalize_contrast(lo, hi, 1 + seed, 255 - 10 * seed, True)
-    np.testing.assert_array_equal(OP.normalize_contrast(img, lo, hi, 1 + seed, 255 - 10 * seed, True), np.asarray(im.array))
     aff = rng.random((3, 4, 12, 10), dtype=np.float32)
-    for mode in ("xy", "z"):
-        np.testing.assert_array_equal(OP.quantize(aff, mode), np.asarray(AffinityMap(aff.copy()).quantize(mode).array))
     mask = rng.integers(0, 2, size=(2, 3, 5), dtype=np.uint8)
-    c = Chunk(aff.copy(), voxel_size=(4, 4, 4))
-    Chunk(mask, voxel_size=(8, 16, 8)).maskout(c)
-    np.testing.assert_array_equal(OP.maskout(mask, (8, 16, 8), aff, (4, 4, 4)), np.asarray(c.array))
-    for margin in ((1, 2, 3), (0, 1, 2, 1, 0, 3)):
-        r = Chunk(aff.copy(), voxel_offset=(3, 2, 1)).crop_margin(margin)
+    return img, (lo, hi, 1 + seed, 255 - 10 * seed, True), aff, mask
+
+
+MARGINS = ((1, 2, 3), (0, 1, 2, 1, 0, 3))
+
+
+@pytest.mark.parametrize("seed", [0, 1, 2])
+def test_against_real_reference(pins, seed):
+    """normalize-contrast, quantize, maskout and crop-margin on fresh random inputs: oracle == the reference's Image /
+    AffinityMap / Chunk methods, bit for bit (recorded by tests/golden/make_golden_reference.py)."""
+    img, nc_args, aff, mask = real_reference_case(seed)
+    pins.exact(f"operators/{seed}/normalize_contrast", OP.normalize_contrast(img, *nc_args))
+    for mode in ("xy", "z"):
+        pins.exact(f"operators/{seed}/quantize_{mode}", OP.quantize(aff, mode))
+    pins.exact(f"operators/{seed}/maskout", OP.maskout(mask, (8, 16, 8), aff, (4, 4, 4)))
+    for k, margin in enumerate(MARGINS):
         a, o = OP.crop_margin(aff, (3, 2, 1), margin)
-        np.testing.assert_array_equal(a, np.asarray(r.array))
-        assert tuple(o) == tuple(r.voxel_offset)
+        pins.exact(f"operators/{seed}/crop_margin/{k}", a)
+        pins.value(f"operators/{seed}/crop_margin/{k}/offset", tuple(o))
 
 
-@pytest.mark.skipif(not H.available(), reason="/root/reference not present (GPU box)")
-def test_normalize_contrast_property_against_real_reference():
-    """Randomised shapes, clip fractions and output ranges (hypothesis, bounded): oracle == real reference, bit for bit,
-    including degenerate histograms (empty, single value, value 255 present / absent)."""
-    from hypothesis import given, settings, strategies as st, HealthCheck
-    H.import_reference()
-    warnings.simplefilter("ignore")
-    from chunkflow.chunk.image.base import Image
-
-    @settings(max_examples=40, deadline=None, suppress_health_check=list(HealthCheck))
-    @given(st.integers(1, 4), st.integers(1, 24), st.integers(1, 24), st.integers(0, 2 ** 31 - 1),
-           st.sampled_from([0.0, 0.01, 0.1, 0.5, 0.9, 1.0]), st.sampled_from([0.0, 0.01, 0.1, 0.5, 1.0]),
-           st.integers(0, 40), st.integers(41, 255), st.sampled_from(["uniform", "dark", "top", "const", "zero"]))
-    def check(z, y, x, seed, lo, hi, mn, mx, kind):
-        rng = np.random.default_rng(seed)
+def normalize_contrast_cases():
+    """Random shapes, clip fractions and output ranges, including degenerate histograms (empty, single value, value 255
+    present / absent)."""
+    rng = np.random.default_rng(85)
+    for k in range(60):
+        z, y, x = int(rng.integers(1, 5)), int(rng.integers(1, 25)), int(rng.integers(1, 25))
+        lo = float(rng.choice([0.0, 0.01, 0.1, 0.5, 0.9, 1.0]))
+        hi = float(rng.choice([0.0, 0.01, 0.1, 0.5, 1.0]))
+        mn, mx = int(rng.integers(0, 41)), int(rng.integers(41, 256))
+        kind = ("uniform", "dark", "top", "const", "zero")[k % 5]
         if kind == "uniform":
             img = rng.integers(0, 256, (z, y, x), dtype=np.uint8)
         elif kind == "dark":
@@ -107,9 +98,10 @@ def test_normalize_contrast_property_against_real_reference():
             img = np.full((z, y, x), rng.integers(0, 256), np.uint8)
         else:
             img = np.zeros((z, y, x), np.uint8)
-        im = Image(img.copy())
-        with redirect_stdout(io.StringIO()), redirect_stderr(io.StringIO()):
-            im.normalize_contrast(lo, hi, mn, mx, True)
-        np.testing.assert_array_equal(OP.normalize_contrast(img, lo, hi, mn, mx, True), np.asarray(im.array))
+        yield img, (lo, hi, mn, mx, True)
 
-    check()
+
+def test_normalize_contrast_property_against_real_reference(pins):
+    """60 seeded random cases (normalize_contrast_cases): oracle == real reference, bit for bit."""
+    for i, (img, args) in enumerate(normalize_contrast_cases()):
+        pins.exact(f"normalize_contrast_random/{i}", OP.normalize_contrast(img, *args))

@@ -265,24 +265,20 @@ def test_plugin_refuses_other_scoring_functions_and_needs_a_gpu():
             agglomerate.execute(affs)
 
 
-def test_plugin_signature_matches_the_reference_plugin():
-    """Same parameter names, order and defaults as chunkflow/plugins/agglomerate.py: execute (read with `ast`: importing the
-    reference module needs waterz), plus the trailing `device` extension; the CLI command carries the same knobs."""
-    import ast
+def test_plugin_signature_matches_the_reference_plugin(pins):
+    """Same parameter names, order and defaults as chunkflow/plugins/agglomerate.py: execute (read with `ast` by
+    tests/golden/make_golden_reference.py: importing the reference module needs waterz), plus the trailing `device`
+    extension; the CLI command carries the same knobs."""
     import inspect
     from chunkflow_b200.flow import cli
     from chunkflow_b200.plugins import agglomerate
+    from reference_pins import REQUIRED, plain
     ours = inspect.signature(agglomerate.execute)
     expected = [("affs", inspect.Parameter.empty), ("fragments", None), ("threshold", 0.7), ("aff_threshold_low", 0.001),
                 ("aff_threshold_high", 0.9999), ("scoring_function", 'OneMinus<MeanAffinity<RegionGraphType, ScoreValue>>'),
                 ("flip_channel", True)]
-    ref_file = "/root/reference/chunkflow/plugins/agglomerate.py"
-    if os.path.exists(ref_file):      # (absent on the GPU box: the list above is what this check read here)
-        fn = next(n for n in ast.parse(open(ref_file).read()).body if isinstance(n, ast.FunctionDef) and n.name == "execute")
-        names = [a.arg for a in fn.args.args]
-        defaults = [ast.literal_eval(d) for d in fn.args.defaults]
-        ref = list(zip(names, [inspect.Parameter.empty] * (len(names) - len(defaults)) + defaults))
-        assert ref == expected
+    assert plain([[n, REQUIRED if d is inspect.Parameter.empty else d] for n, d in expected]) == \
+        pins.get("agglomerate/execute_signature")
     got = [(n, p.default) for n, p in ours.parameters.items()]
     assert got[:len(expected)] == expected and [n for n, _ in got[len(expected):]] == ["device"]
     opts = {o for p in cli.agglomerate.params for o in p.opts + p.secondary_opts}
