@@ -16,7 +16,7 @@ OK = 0
 ERR_INVALID_ARGUMENT, ERR_CUDA, ERR_WEIGHTS, ERR_OUTPUT_RANGE, ERR_UNSUPPORTED, ERR_CAPACITY = -1, -2, -3, -4, -5, -6
 FRAMEWORK_UNET3L, FRAMEWORK_IDENTITY = 0, 1
 PRECISION_F32_SIMT, PRECISION_F16X3_UMMA, PRECISION_F16_UMMA, PRECISION_F16F8_UMMA = 0, 1, 2, 3
-DTYPE_U8, DTYPE_F32, DTYPE_U32 = 0, 1, 2
+DTYPE_U8, DTYPE_F32, DTYPE_U32, DTYPE_U64 = 0, 1, 2, 3
 AUGMENT_NONE, AUGMENT_REFERENCE, AUGMENT_SPATIAL = 0, 1, 2
 QUANTIZE_XY, QUANTIZE_Z = 0, 1
 
@@ -32,6 +32,7 @@ EXPORTS = (
     "cfb_connected_components_device", "cfb_connected_components_workspace",
     "cfb_watershed_workspace", "cfb_watershed_device", "cfb_region_graph_workspace", "cfb_region_graph_device",
     "cfb_region_graph_read", "cfb_agglomerate_edges_host", "cfb_relabel_device",
+    "cfb_contingency_workspace", "cfb_contingency_device", "cfb_contingency_scores", "cfb_contingency_read",
 )
 
 
@@ -44,6 +45,13 @@ class Params(C.Structure):
         ("mask_output_chunk", C.c_int32), ("augment", C.c_int32), ("has_myelin_threshold", C.c_int32),
         ("mask_myelin_threshold", C.c_float), ("check_output_range", C.c_int32),
     ]
+
+
+class ContingencySums(C.Structure):
+    """cfb_contingency_sums (include/chunkflow_b200.h)."""
+    _fields_ = [(n, C.c_uint64) for n in ("voxels", "entries", "sum_sq_pairs", "sum_sq_seg", "sum_sq_gt", "nonzero_voxels",
+                                          "seg_labels", "pairs_over_threshold")] + \
+               [(n, C.c_uint64 * 2) for n in ("xlogx_pairs", "xlogx_seg", "xlogx_gt")]
 
 
 class NativeError(RuntimeError):
@@ -126,6 +134,11 @@ def load() -> C.CDLL:
     lib.cfb_region_graph_read.argtypes = [vp, i64, i64, vp, vp, vp, vp, vp]
     lib.cfb_agglomerate_edges_host.argtypes = [i64, i64, vp, vp, vp, vp, C.c_float, vp]
     lib.cfb_relabel_device.argtypes = [vp, i64, vp, i64, vp, vp]
+    lib.cfb_contingency_workspace.argtypes = [i64]
+    lib.cfb_contingency_workspace.restype = i64
+    lib.cfb_contingency_device.argtypes = [vp, i32, vp, i32, i64, vp, i64, C.POINTER(i64), vp]
+    lib.cfb_contingency_scores.argtypes = [vp, i64, i64, i64, C.c_double, C.POINTER(ContingencySums), vp]
+    lib.cfb_contingency_read.argtypes = [vp, i64, i64, vp, vp, vp, vp]
     for name in EXPORTS:
         getattr(lib, name)   # every declared symbol must be there
     _lib = lib
@@ -230,6 +243,48 @@ def agglomerate_edges_host(num_nodes: int, u, v, sum_fixed, count, threshold: fl
 def relabel_device(d_labels: int, n: int, d_map: int, map_size: int, d_out: int, stream: int = 0) -> None:
     check(load().cfb_relabel_device(C.c_void_p(d_labels), int(n), C.c_void_p(d_map), int(map_size), C.c_void_p(d_out),
                                     C.c_void_p(stream)))
+
+
+# ---- `evaluate-segmentation` (include/chunkflow_b200.h) ----
+def contingency_workspace(table_slots: int) -> int:
+    return int(load().cfb_contingency_workspace(int(table_slots)))
+
+
+def _check_slots(table_slots: int, d_workspace_bytes: Optional[int]) -> None:
+    if table_slots < 2 or table_slots & (table_slots - 1):
+        raise ValueError("table_slots must be a power of two")
+    if d_workspace_bytes is not None and d_workspace_bytes < contingency_workspace(table_slots):
+        raise ValueError(f"the workspace holds {d_workspace_bytes} bytes; {table_slots} slots need {contingency_workspace(table_slots)}")
+
+
+def contingency_device(d_seg: int, seg_dtype: int, d_gt: int, gt_dtype: int, n: int, d_workspace: int, table_slots: int,
+                       workspace_bytes: Optional[int] = None, stream: int = 0) -> int:
+    """-> number of (seg id, gt id) pairs; raises NativeError with code ERR_CAPACITY when the table is too small."""
+    _check_slots(table_slots, workspace_bytes)
+    e = C.c_int64()
+    check(load().cfb_contingency_device(C.c_void_p(d_seg), int(seg_dtype), C.c_void_p(d_gt), int(gt_dtype), int(n), C.c_void_p(d_workspace),
+                                        int(table_slots), C.byref(e), C.c_void_p(stream)))
+    return int(e.value)
+
+
+def contingency_scores(d_workspace: int, table_slots: int, n: int, num_entries: int, size_threshold: float,
+                       workspace_bytes: Optional[int] = None, stream: int = 0) -> ContingencySums:
+    _check_slots(table_slots, workspace_bytes)
+    out = ContingencySums()
+    check(load().cfb_contingency_scores(C.c_void_p(d_workspace), int(table_slots), int(n), int(num_entries), float(size_threshold),
+                                        C.byref(out), C.c_void_p(stream)))
+    return out
+
+
+def contingency_read(d_workspace: int, table_slots: int, num_entries: int, workspace_bytes: Optional[int] = None, stream: int = 0):
+    """-> (seg_ids, gt_ids, counts) uint64 host arrays sorted by (seg id, gt id)."""
+    _check_slots(table_slots, workspace_bytes)
+    if not 0 <= num_entries <= table_slots // 2:
+        raise ValueError("num_entries does not fit the table")
+    s, g, c = (np.empty(int(num_entries), np.uint64) for _ in range(3))
+    check(load().cfb_contingency_read(C.c_void_p(d_workspace), int(table_slots), int(num_entries), _ptr(s), _ptr(g), _ptr(c),
+                                      C.c_void_p(stream)))
+    return s, g, c
 
 
 def device_memory(device: int = 0) -> tuple:

@@ -11,6 +11,7 @@ bookkeeping of the reference's ``Chunk`` and mirrors, name for name, the referen
     quantize             reference chunk/affinity_map/base.py:33-57     (AffinityMap)
     connected_component  reference chunk/base.py:128-137                (Chunk -> cc3d)
     agglomerate          reference plugins/agglomerate.py:8-48          (plugin -> waterz)
+    evaluate             reference chunk/segmentation.py:33-67          (Segmentation -> gala)
 
 so that ``create-chunk | normalize-contrast | inference | crop-margin | quantize`` moves the image to the GPU once and
 brings a uint8 thumbnail (or nothing) back instead of the 12-byte-per-voxel affinity map.  There is no CPU fallback.
@@ -68,6 +69,9 @@ def mask_array_for(chunk_dtype, mask: np.ndarray) -> np.ndarray:
     raise TypeError(f"unsupported chunk dtype {chunk_dtype}")
 
 
+EVALUATE_INITIAL_SLOTS = 1 << 20   # contingency-table slots of the first attempt; grown eightfold while the pairs overflow it
+
+
 class DeviceChunk:
     def __init__(self, tensor, voxel_offset=None, voxel_size=None, layer_type: Optional[str] = None):
         torch = _torch()
@@ -94,6 +98,15 @@ class DeviceChunk:
         target = np.uint8 if like.tensor.dtype == torch.uint8 else np.float32
         arr = mask_array_for(target, mask.array)
         return cls(torch.from_numpy(arr).to(like.tensor.device), voxel_offset=mask.voxel_offset, voxel_size=mask.voxel_size)
+
+    @classmethod
+    def from_labels(cls, labels: np.ndarray, device="cuda:0", voxel_offset=None, voxel_size=None) -> "DeviceChunk":
+        """A (z,y,x) uint32 / uint64 label volume, uploaded as int32 / int64 with the same bits (torch's unsigned types
+        have few operations)."""
+        torch = _torch()
+        signed = {np.dtype(np.uint32): np.int32, np.dtype(np.uint64): np.int64}[np.dtype(labels.dtype)]
+        t = torch.from_numpy(np.ascontiguousarray(labels).view(signed)).to(device)
+        return cls(t, voxel_offset=voxel_offset, voxel_size=voxel_size, layer_type="segmentation")
 
     def to_chunk(self) -> Chunk:
         return Chunk(self.tensor.cpu().numpy(), voxel_offset=self.voxel_offset, voxel_size=self.voxel_size)
@@ -304,6 +317,71 @@ class DeviceChunk:
         out.num_fragments, out.num_edges = num, int(u.size)
         out.num_components = int(np.count_nonzero(root[1:] == np.arange(1, root.size, dtype=np.uint32)))
         return out
+
+    # ---- Segmentation.evaluate (reference chunk/segmentation.py:33-67 -> lib/gala/evaluate.py) ------------------------
+    def _label_tensor(self, what: str):
+        """The labels as a contiguous 4- or 8-byte tensor and its native dtype code; ids are read as unsigned, narrower
+        integer types are widened (bijections that keep 0 change no score)."""
+        torch = _torch()
+        t = self.tensor
+        if t.ndim == 4:
+            if t.shape[0] != 1:
+                raise ValueError(f"{what}: a segmentation has one channel, not {t.shape[0]}")
+            t = t[0]
+        if t.is_floating_point() or t.is_complex():
+            raise TypeError(f"{what} must be an integer label volume, not {t.dtype}")
+        if t.element_size() < 4:
+            t = t.to(torch.int32)
+        t = t.contiguous()
+        if t.data_ptr() % 16:
+            t = t.clone()
+        return t, (_native.DTYPE_U64 if t.element_size() == 8 else _native.DTYPE_U32)
+
+    def _contingency(self, groundtruth: "DeviceChunk"):
+        """Builds the contingency table of (self, groundtruth) on the device -> (workspace, slots, entries, voxels)."""
+        torch = _torch()
+        s, s_code = self._label_tensor("the segmentation")
+        g, g_code = groundtruth._label_tensor("the ground truth")
+        if tuple(s.shape) != tuple(g.shape):
+            raise ValueError(f"the ground truth has shape {tuple(g.shape)}, the segmentation {tuple(s.shape)}")
+        if s.device != g.device:
+            raise ValueError("the segmentation and the ground truth must be on the same GPU")
+        n = s.numel()
+        slots = EVALUATE_INITIAL_SLOTS
+        most = 4
+        while most < 2 * n:   # a table never holds more pairs than voxels
+            most <<= 1
+        slots = max(2, min(slots, most))
+        with self._on_device():
+            while True:
+                work = torch.empty(_native.contingency_workspace(slots), dtype=torch.uint8, device=s.device)
+                try:
+                    entries = _native.contingency_device(s.data_ptr(), s_code, g.data_ptr(), g_code, n, work.data_ptr(), slots,
+                                                         work.numel(), self._stream())
+                    return work, slots, entries, n
+                except _native.NativeError as err:
+                    if err.code != _native.ERR_CAPACITY or slots >= most:
+                        raise
+                del work
+                slots = min(slots << 3, most)   # more pairs than half the slots: a larger table
+
+    def evaluate(self, groundtruth: "DeviceChunk", size_threshold: float = 1000) -> dict:
+        """The reference's ``Segmentation.evaluate`` dict (``rand_index``, ``adjusted_rand_index``,
+        ``variation_of_information``, ``fowlkes_mallows_index``, ``edit_distance``) of this segmentation against
+        ``groundtruth``, both (z,y,x) integer volumes on the same GPU.  One pass over both volumes builds the contingency
+        table; a reduction on the device turns it into exact integer sums; the scores are finished on the host."""
+        from .segmentation import scores_from_sums
+        work, slots, entries, n = self._contingency(groundtruth)
+        with self._on_device():
+            sums = _native.contingency_scores(work.data_ptr(), slots, n, entries, float(size_threshold), work.numel(), self._stream())
+        return scores_from_sums(sums)
+
+    def contingency_table(self, groundtruth: "DeviceChunk"):
+        """(seg_ids, gt_ids, counts) uint64 host arrays: the number of voxels of every label pair that occurs, sorted by
+        (seg id, gt id); signed ids appear as their unsigned bit patterns."""
+        work, slots, entries, _ = self._contingency(groundtruth)
+        with self._on_device():
+            return _native.contingency_read(work.data_ptr(), slots, entries, work.numel(), self._stream())
 
     def __repr__(self):
         return f"DeviceChunk(shape={self.shape}, dtype={self.dtype}, voxel_offset={tuple(self.voxel_offset)}, device={self.tensor.device})"

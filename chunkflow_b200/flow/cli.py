@@ -301,5 +301,52 @@ def agglomerate(tasks, name, input_chunk_name, output_chunk_name, threshold, aff
         yield task
 
 
+@main.command("load-npy")
+@click.option("--file-name", "-f", type=click.Path(exists=True, file_okay=True, dir_okay=False, readable=True, resolve_path=True),
+              required=True, help="file name path")
+@click.option("--voxel-offset", "-t", type=int, nargs=3, default=(0, 0, 0), help="voxel offset")
+@click.option("--voxel-size", "-s", type=click.FLOAT, nargs=3, default=(1, 1, 1), help="voxel size")
+@click.option("--output-name", "-o", type=str, default="chunk", help="output name in the task dictionary.")
+@operator
+def load_npy(tasks, file_name, voxel_offset, voxel_size, output_name):
+    """Load a chunk from a .npy file (reference flow/flow.py:1321-1341), e.g. a ground truth for `evaluate-segmentation`."""
+    for task in tasks:
+        if task is not None:
+            if not file_name.endswith(".npy"):
+                raise click.BadParameter(f"{file_name} is not a .npy file", param_hint="--file-name")
+            task[output_name] = Chunk(np.load(file_name), voxel_offset=voxel_offset, voxel_size=voxel_size)
+        yield task
+
+
+@main.command("evaluate-segmentation")
+@click.option("--segmentation-chunk-name", "-s", type=str, default="chunk", help="chunk name of segmentation")
+@click.option("--groundtruth-chunk-name", "-g", type=str, default="groundtruth")
+@click.option("--output", "-o", type=str, default="seg_score", help="segmentation evaluation result name.")
+@operator
+def evaluate_segmentation(tasks, segmentation_chunk_name, groundtruth_chunk_name, output):
+    """Score a segmentation against a ground truth: Rand index, adjusted Rand index, variation of information,
+    Fowlkes-Mallows index, edit distance (reference flow/flow.py:1519-1542, chunk/segmentation.py:33-67).  Either chunk may
+    be on the host or, after `to-device`, on the GPU; the contingency table is built on the GPU either way."""
+    from chunkflow_b200.chunk.device import DeviceChunk
+    from chunkflow_b200.chunk.segmentation import Segmentation, format_scores
+    for task in tasks:
+        if task is not None:
+            seg, gt = task[segmentation_chunk_name], task[groundtruth_chunk_name]
+            if isinstance(seg, Chunk) and isinstance(gt, Chunk):
+                task[output] = Segmentation(seg.array, voxel_offset=seg.voxel_offset).evaluate(gt)
+            else:
+                dev = seg if isinstance(seg, DeviceChunk) else gt
+                seg, gt = (c if isinstance(c, DeviceChunk) else _device_labels(c, dev.tensor.device) for c in (seg, gt))
+                task[output] = seg.evaluate(gt)
+                print(format_scores(task[output]), end="")
+        yield task
+
+
+def _device_labels(chunk, device):
+    from chunkflow_b200.chunk.device import DeviceChunk
+    from chunkflow_b200.chunk.segmentation import label_array
+    return DeviceChunk.from_labels(label_array(chunk.array, "a label chunk"), device=device)
+
+
 if __name__ == "__main__":
     main()

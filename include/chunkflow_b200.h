@@ -73,6 +73,7 @@ extern "C" {
 #define CFB_DTYPE_U8 0
 #define CFB_DTYPE_F32 1
 #define CFB_DTYPE_U32 2 /* connected components on an integer segmentation */
+#define CFB_DTYPE_U64 3 /* label volumes of evaluate-segmentation */
 
 typedef struct cfb_engine* cfb_handle;
 
@@ -294,6 +295,43 @@ int cfb_agglomerate_edges_host(int64_t num_nodes, int64_t num_edges, const uint3
 /* d_out[i] = d_map[d_labels[i]] (labels >= map_size pass through): applies root_of to the fragments. */
 int cfb_relabel_device(const uint32_t* d_labels, int64_t n, const uint32_t* d_map, int64_t map_size, uint32_t* d_out,
                        void* stream);
+
+/* `evaluate-segmentation` (reference flow/flow.py:1519-1542 -> chunk/segmentation.py:33-67 -> lib/gala/evaluate.py).
+ *
+ * cfb_contingency_device: one pass over d_seg and d_gt (n voxels each, CFB_DTYPE_U32 or CFB_DTYPE_U64, 16-byte aligned; every
+ * id is a label, 0 and 2^64 - 1 included) builds the contingency table -- the number of voxels of every (seg id, gt id) pair
+ * that occurs -- with exact 64-bit counts in an open-addressing table of `table_slots` (a power of two) slots inside
+ * d_workspace (cfb_contingency_workspace(table_slots) bytes).  *num_entries = pairs found.  Returns CFB_ERR_CAPACITY when the
+ * pairs fill more than half the slots: call again with a larger table.  Synchronises the stream.
+ *
+ * cfb_contingency_scores: reduces the table (the workspace of a successful cfb_contingency_device) to the exact integer sums
+ * below, in the same number whatever the order of the device's atomics.  Synchronises the stream.
+ *
+ * cfb_contingency_read: copies the table to the host, sorted by (seg id, gt id). */
+typedef struct cfb_contingency_sums {
+  uint64_t voxels;               /* n */
+  uint64_t entries;              /* pairs (s, g) in the table */
+  uint64_t sum_sq_pairs;         /* sum of n_sg^2 over the table */
+  uint64_t sum_sq_seg;           /* sum of a_s^2, a_s = sum_g n_sg (label 0 included) */
+  uint64_t sum_sq_gt;            /* sum of b_g^2, b_g = sum_s n_sg */
+  uint64_t nonzero_voxels;       /* voxels with s != 0 and g != 0 */
+  uint64_t seg_labels;           /* distinct s != 0 */
+  uint64_t pairs_over_threshold; /* pairs with s != 0, g != 0 and n_sg > size_threshold */
+  /* sums of x log2 x in 128-bit fixed point with 62 fractional bits, {low word, high word}; each term is a double,
+   * converted exactly; terms with label 0 on either side left out:
+   * over n_sg (s != 0, g != 0); over a'_s = sum_{g != 0} n_sg (s != 0); over b'_g = sum_{s != 0} n_sg (g != 0) */
+  uint64_t xlogx_pairs[2];
+  uint64_t xlogx_seg[2];
+  uint64_t xlogx_gt[2];
+} cfb_contingency_sums;
+
+int64_t cfb_contingency_workspace(int64_t table_slots);
+int cfb_contingency_device(const void* d_seg, int32_t seg_dtype, const void* d_gt, int32_t gt_dtype, int64_t n, void* d_workspace,
+                           int64_t table_slots, int64_t* num_entries, void* stream);
+int cfb_contingency_scores(void* d_workspace, int64_t table_slots, int64_t n, int64_t num_entries, double size_threshold,
+                           cfb_contingency_sums* out, void* stream);
+int cfb_contingency_read(void* d_workspace, int64_t table_slots, int64_t num_entries, uint64_t* h_seg, uint64_t* h_gt,
+                         uint64_t* h_count, void* stream);
 
 #ifdef __cplusplus
 }
